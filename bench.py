@@ -13,7 +13,13 @@ layer-direction of CogVideoX-5B (48 heads x 64, mini-batch 64, checkpoint group 
                     keys: single-sequence latency through the chain, and plain data-parallel replicas.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--mode fwd|fwdbwd] [--nc 5487] [--batch 1] [--seqs M]
+                    [--dump-outputs DIR]
     python bench.py --impl reference ...      # the reference's eager CPU path on the host cores
+
+--dump-outputs DIR writes what the last timed step handed back to its caller as DIR/<name>.npy (float32): the op's output
+`out` and, in fwd+bwd mode, the token gradients dXQ/dXK/dXV and the parameter gradients.  The inputs are seeded, so two builds
+run with the same arguments can be compared array by array.  An array of more than DUMP_ELEMS elements is reduced to a fixed,
+seeded sample of rows of its last dimension (the same rows for every array of the same shape).
 
 value   = tokens/s with inputs resident in HBM (CUDA-event time, max over ranks, whole-job aggregate)
 e2e     = same through the public op with HOST (pinned) inputs: H2D of q,k,v,eta(,dOut) + op + D2H of the op's output per
@@ -31,6 +37,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark may run from a read-only tree and leaves nothing behind in it
 os.environ.setdefault("TORCHDYNAMO_DISABLE", "1")
 
 U_FLOP = 2 * 64 * 64 * 256
@@ -38,12 +45,15 @@ FWD_U, BWD_U = 7, 15
 H_5B = 48
 NC_63S, NC_9S, NC_3S = 5487, 804, 282
 CPU_SAMPLE_NC = 64  # BASELINE.md section 3: time a prefix of >= 64 mini-batches, the scan cost is linear in NC
+PARAM_NAMES = ("ln_w", "ln_b", "W1", "b1", "W2", "b2")
+DUMP_ELEMS = 1 << 20  # per dumped array (4 MB in float32): at most 10 arrays stay well inside 64 MB
+DUMP_SEED = 0
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--mode", default="fwdbwd", choices=["auto", "fwd", "fwdbwd"])
@@ -56,7 +66,12 @@ def parse():
                     help="N>1: sequence-sharded chain (default) or independent data-parallel replicas")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary keys (nc804 / latency / replicas)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (un-sharded runs; rank 0)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 def peaks():
@@ -105,30 +120,17 @@ def usable_cores():
 
 
 class CpuEager:
-    """The reference's eager CPU path of the op on a bounded sample: the real `ttt.models.ssm.ops.ttt_mlp` when
-    /root/reference is importable (kind "reference": the build container), else its restatement oracle/ttt_oracle.py (kind
-    "port": the GPU box, where /root/reference does not exist).  fp32, eta materialised [.., CS, CS] as the reference does
-    (ttt_layer.py:288), autograd backward."""
+    """The reference's eager CPU path of the op on a bounded sample, as restated in oracle/ttt_oracle.py (kind "port"; the
+    restatement is pinned to the reference's outputs by tests/test_oracle.py).  fp32, eta materialised [.., CS, CS] as the
+    reference does (ttt_layer.py:288), autograd backward."""
 
     def __init__(self, heads, mode, sample_nc=CPU_SAMPLE_NC):
         import torch
         from oracle import ttt_oracle as O
         self.torch, self.mode, self.heads, self.nc = torch, mode, heads, sample_nc
         self.d = O.make_inputs(1, heads, sample_nc, seed=0)
-        self.kind, self.fn = "port", None
-        ref_root = "/root/reference"
-        if os.path.isdir(os.path.join(ref_root, "ttt", "models", "ssm")):
-            try:
-                sys.path.insert(0, ref_root)
-                from ttt.models.ssm.ops import ttt_mlp as ref_ttt_mlp  # ttt/models/ssm/ops/ttt_mlp.py:70
-                self.kind = "reference"
-                self.fn = lambda k, q, v, e, lw, lb, W1, b1, W2, b2: ref_ttt_mlp(k, q, v, e, lw, lb, W1, b1, W2, b2, 16)
-            except Exception:
-                self.kind, self.fn = "port", None
-            finally:
-                sys.path.remove(ref_root)
-        if self.fn is None:
-            self.fn = lambda *a: O.ttt_mlp_eager(*a)[0]
+        self.kind = "port"
+        self.fn = lambda *a: O.ttt_mlp_eager(*a)[0]
 
     def once(self):
         torch, d = self.torch, self.d
@@ -172,7 +174,7 @@ class CpuEager:
 
     def describe(self, threads):
         return (f"first {self.nc} mini-batches ({self.nc * 64} tokens) x {self.heads} heads, fp32 eager dual form "
-                f"({'ttt.models.ssm.ops.ttt_mlp of /root/reference' if self.kind == 'reference' else 'oracle port of ttt/models/ssm/ops/ttt_mlp.py'}), "
+                f"(oracle port of ttt/models/ssm/ops/ttt_mlp.py), "
                 f"{'fwd' if self.mode == 'fwd' else 'fwd + autograd bwd'}, {threads} threads = fastest of 1..{usable_cores()} usable cores, "
                 f"median of the timed passes after one warm-up")
 
@@ -265,27 +267,59 @@ def max_over_ranks(torch, dist, world, dev, *vals):
     return [float(x) for x in t]
 
 
-def single_gpu_op(torch, mlp_tk, params, mode, G):
+def single_gpu_op(torch, mlp_tk, params, mode, G, outputs=None):
     def step(q, k, v, e, go):
-        """One pass of the hot path through the public op (TkMLP.apply-compatible entry, last-row eta form)."""
+        """One pass of the hot path through the public op (TkMLP.apply-compatible entry, last-row eta form).  `outputs`, when
+        given, holds what the pass hands back to its caller until the next pass starts."""
+        if outputs is not None:
+            outputs.clear()
         if mode == "fwdbwd":
+            for p in params:  # each pass leaves its own parameter gradients, as a training step does
+                p.grad = None
             q = q.detach().requires_grad_(True); k = k.detach().requires_grad_(True); v = v.detach().requires_grad_(True)
         out = mlp_tk.ttt_mlp_op(*params, q, v, k, e, G)
         if mode == "fwdbwd":
             out.backward(go)
+        if outputs is not None:
+            outputs["out"] = out
+            if mode == "fwdbwd":
+                outputs.update(dXQ=q.grad, dXK=k.grad, dXV=v.grad, **{"d" + n: p.grad for n, p in zip(PARAM_NAMES, params)})
         return out
     return step
 
 
-def bench_replica(args, torch, dist, mlp_tk, world, rank, dev, mode, NC, with_e2e, steps, warmup, sampler=None):
-    """B sequences per GPU, un-sharded: the N = 1 workload, and the data-parallel-replica secondary key at N > 1."""
+def dump_outputs(torch, outputs, path):
+    """Each array as path/<name>.npy in float32; one of more than DUMP_ELEMS elements as the rows (of its last dimension) at
+    DUMP_ELEMS // last_dim indices drawn with a fixed seed, in ascending order."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    total = 0
+    for name, t in outputs.items():
+        t = t.detach().reshape(-1, t.shape[-1])
+        if t.numel() > DUMP_ELEMS:
+            g = torch.Generator().manual_seed(DUMP_SEED)
+            rows = torch.randint(t.shape[0], (DUMP_ELEMS // t.shape[1],), generator=g).sort().values
+            t = t[rows.to(t.device)]
+        a = t.float().cpu().numpy()
+        np.save(os.path.join(path, name + ".npy"), a)
+        total += a.nbytes
+    assert total <= 64 << 20, total
+
+
+def bench_replica(args, torch, dist, mlp_tk, world, rank, dev, mode, NC, with_e2e, steps, warmup, sampler=None, dump=None):
+    """B sequences per GPU, un-sharded: the N = 1 workload, and the data-parallel-replica secondary key at N > 1.  `dump`: a
+    directory that receives this rank's outputs of the last timed step."""
     B, H, G = args.batch, args.heads, args.ckpt
     params = synth_params(torch, dev, B, H)
     if mode == "fwdbwd":
         params = [p.requires_grad_(True) for p in params]
     q, k, v, e, go = synth(torch, dev, B, H, NC, 1234 + rank, mode == "fwdbwd")
-    step = single_gpu_op(torch, mlp_tk, params, mode, G)
+    outputs = {} if dump else None
+    step = single_gpu_op(torch, mlp_tk, params, mode, G, outputs)
     ms = timed(torch, dist, world, lambda: step(q, k, v, e, go), steps, warmup, sampler)
+    if dump:
+        dump_outputs(torch, outputs, dump)
+        outputs.clear()
     res = {"ms_per_step": ms / steps, "tokens_per_step": B * NC * 64 * world,
            "launches": steps * mlp_tk.launches_per_call(mode)}
     if with_e2e:
@@ -495,29 +529,28 @@ def main():
 
     import torch
     import torch.distributed as dist
-    import __graft_entry__
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    sharded = world > 1 and args.parallel in ("auto", "seqshard")
+    if args.dump_outputs and sharded:
+        sys.exit("bench.py: --dump-outputs needs an un-sharded run (one GPU, or --parallel replicas)")
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
-    if rank == 0:
-        __graft_entry__.build()
-    if world > 1:
-        dist.barrier()
-    from ttt_video_dit_b200 import mlp_tk
+    from ttt_video_dit_b200 import _lib, mlp_tk
+    _lib.lib()  # the library build() made; raises if it is missing (the benchmark compiles nothing into the tree)
 
     mode = "fwd" if args.mode == "fwd" else "fwdbwd"
     H, NC, G = args.heads, args.nc, args.ckpt
-    sharded = world > 1 and args.parallel in ("auto", "seqshard")
     M = (args.seqs or 8 * world) if sharded else None
     sampler = ClockSampler(local)
     if sharded:
         r = bench_sharded(args, torch, dist, world, rank, dev, mode, NC, M, True, args.steps, args.warmup, sampler)
     else:
-        r = bench_replica(args, torch, dist, mlp_tk, world, rank, dev, mode, NC, True, args.steps, args.warmup, sampler)
+        r = bench_replica(args, torch, dist, mlp_tk, world, rank, dev, mode, NC, True, args.steps, args.warmup, sampler,
+                          dump=args.dump_outputs if rank == 0 else None)
     ms_step, ms_e2e = max_over_ranks(torch, dist, world, dev, r["ms_per_step"], r["e2e_ms_per_step"])
 
     secondary = {}

@@ -1,17 +1,20 @@
-"""Generate tests/golden/*.pt by RUNNING THE UNMODIFIED REFERENCE (build container only).
+"""Generate tests/golden/*.pt by RUNNING THE UNMODIFIED REFERENCE (a checkout of the original ttt-video-dit project).
 
-    TORCHDYNAMO_DISABLE=1 PYTHONPATH=/root/reference python oracle/make_golden.py
+    TORCHDYNAMO_DISABLE=1 TTT_VIDEO_DIT_ROOT=<checkout> python oracle/make_golden.py \
+        [integration_patch|sampling|transformer_layer|process_input|layer]
 
 Each fixture holds the reference's outputs (fp64, CPU, true eager) for seeded inputs that
 ``oracle.ttt_oracle.make_inputs`` regenerates bit-identically from the stored seed; an input
 checksum guards against RNG drift.  The script also asserts that the oracle restatement agrees
 with the reference before anything is written, so a committed fixture == "oracle pinned".
 
-Reference entry points exercised (file:line in /root/reference):
+Reference entry points exercised (file:line in the checkout):
   ttt/models/ssm/ops/ttt_mlp.py:70      ttt_mlp      (+ torch autograd => gradient oracle)
   ttt/models/ssm/ops/ttt_linear.py:57   ttt_linear
   ttt/models/cogvideo/dit.py:224-266    SeqModelingBlock._ssm_forward (gate / flip / reverse)
   ttt/models/cogvideo/dit.py:163-211    SeqModelingBlock._attn_forward (local attention)
+  ttt/models/cogvideo/utils.py:460-492  DiscreteDenoiser.forward (per-element guidance loop)
+  integration/ttt_video_dit_b200.patch  applied to the checkout (hashes of the lines it replaces, CPU path unchanged)
 """
 import os
 import sys
@@ -20,7 +23,9 @@ os.environ.setdefault("TORCHDYNAMO_DISABLE", "1")
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
-sys.path.insert(0, "/root/reference")
+REF = os.environ.get("TTT_VIDEO_DIT_ROOT")
+if REF:
+    sys.path.insert(0, REF)
 
 import torch
 
@@ -336,8 +341,114 @@ def gen_transformer_layer():
     torch.save(out, os.path.join(GOLD, "transformer_layer_ref.pt"))
 
 
+def sampling_network(calls):
+    """Stand-in for the DiT in the denoiser fixture: per-element results do not depend on the batching; records the batch size
+    of every call.  tests/test_sampling_host.py restates it."""
+    def network(x, crossattn, c_noise):
+        calls.append(x.shape[0])
+        return torch.tanh(x) * (1 + 0.01 * c_noise.float().reshape(-1, 1, 1, 1, 1)) + crossattn.mean(dim=(1, 2)).reshape(-1, 1, 1, 1, 1)
+    return network
+
+
+def gen_sampling():
+    """The reference's DiscreteDenoiser.forward (utils.py:460-492) on a classifier-free-guidance pair, fp32 on CPU: its output,
+    the batch size of each network call it makes, and its discretisation table."""
+    from ttt.models.cogvideo import utils as RU
+    torch.manual_seed(0)
+    calls = []
+    ref = RU.DiscreteDenoiser.__new__(RU.DiscreteDenoiser)
+    torch.nn.Module.__init__(ref)
+    ref.scaling = RU.VideoScaling()
+    ref.sigmas = RU.ZeroSNRDDPMDiscretization()(1000, do_append_zero=False, device="cpu", flip=True)
+    ref.quantize_c_noise, ref.network, ref.dtype = True, sampling_network(calls), torch.float32
+    x = torch.randn(2, 3, 4, 5, 6)
+    crossattn = torch.randn(2, 7, 8)
+    step = 400
+    with torch.no_grad():
+        out = ref(x, ref.sigmas[[step, step]].clone(), {"crossattn": crossattn}, idx=ref.sigmas[[step, step]])
+    print("sampling ok, network calls", calls)
+    torch.save(dict(sigmas=ref.sigmas.clone(), x=x, crossattn=crossattn, step=step, calls=calls, out=out),
+               os.path.join(GOLD, "sampling_ref.pt"))
+
+
+PATCH_SCRIPT = r'''
+import sys, torch
+torch.manual_seed(0)
+from ttt.models.cogvideo.dit import SeqModelingBlock
+from ttt.models.cogvideo.utils import SequenceMetadata
+from ttt.models.configs import ModelConfig
+import ttt.models.ssm.ttt_layer as TL
+print("TKMLP", TL.TkMLP.__module__, "LINEAR", TL.TritonLinear.__module__)
+E, NH, Hh, Ww, frames, T, chunks = 128, 2, 4, 4, 25, 8, 2
+cfg = ModelConfig(model_dim=E, num_heads=NH, num_layers=1, ssm_layer="ttt_linear", mini_batch_size=16, ttt_base_lr=1.0,
+                  latent_height=Hh, latent_width=Ww, compressed_num_frames=frames, adapter_method="sft")
+blk = SeqModelingBlock(cfg).double()
+class Stub(torch.nn.Module):
+    def forward(self, x, seq_metadata):
+        return torch.cumsum(x, dim=1) * 0.01 + torch.roll(x, 1, dims=-1) * 0.5
+blk.ssm = Stub()
+md = SequenceMetadata(text_length=T, seq_text_length=T * chunks, num_frames=frames, num_chunks=chunks, tokens_per_frame=Hh * Ww,
+                      latent_height=Hh, latent_width=Ww, t_emb=torch.zeros(1, 8))
+md.init_multiscene_offsets()
+vid = torch.randn(2, frames * Hh * Ww, E, dtype=torch.float64)
+txt = torch.randn(2, T * chunks, E, dtype=torch.float64)
+with torch.no_grad():
+    a = blk._attn_forward(vid, txt, md)
+    s = blk._ssm_forward(torch.cat((txt, vid), dim=1), md)
+print("SUM %.12e %.12e" % (a.double().sum().item(), s.double().sum().item()))
+'''
+
+
+def gen_integration_patch():
+    """integration/ttt_video_dit_b200.patch against the checkout: `patch -p1` applies it without offset or fuzz, the patched
+    tree binds TkMLP / TritonLinear to this package, and a SeqModelingBlock (attention + gate/flip, fp64 on CPU) gives
+    bit-identical results patched and stock.  Records the patch's sha256, for every hunk the sha256 of the lines it replaces
+    in the checkout, and the two runs' results (tests/test_integration_patch.py)."""
+    import json
+    import shutil
+    import subprocess
+    import tempfile
+    from oracle import patch_hunks
+    patch_path = os.path.join(ROOT, "integration", "ttt_video_dit_b200.patch")
+    text = open(patch_path).read()
+
+    def run(pythonpath):
+        env = dict(os.environ, TORCHDYNAMO_DISABLE="1", PYTHONPATH=os.pathsep.join(pythonpath))
+        r = subprocess.run([sys.executable, "-c", PATCH_SCRIPT], capture_output=True, text=True, env=env, timeout=900)
+        assert r.returncode == 0, r.stderr[-3000:]
+        return [l for l in r.stdout.splitlines() if l.startswith(("TKMLP", "SUM"))]
+    with tempfile.TemporaryDirectory() as tmp:
+        shutil.copytree(os.path.join(REF, "ttt"), os.path.join(tmp, "ttt"))
+        r = subprocess.run(["patch", "-p1", "--no-backup-if-mismatch", "-i", patch_path], cwd=tmp, capture_output=True, text=True)
+        assert r.returncode == 0 and "offset" not in r.stdout and "fuzz" not in r.stdout, r.stdout + r.stderr
+        patched = run([tmp, ROOT])
+    stock = run([REF])
+    assert patched[0] == "TKMLP ttt_video_dit_b200.mlp_tk LINEAR ttt_video_dit_b200.linear_triton", patched
+    assert stock[0] == "TKMLP ttt.models.ssm.mlp_tk LINEAR ttt.models.ssm.linear_triton", stock
+    assert patched[1] == stock[1], (patched, stock)
+    files = {}
+    for path, hunks in patch_hunks.parse(text).items():
+        lines = open(os.path.join(REF, path)).read().splitlines()
+        files[path] = [dict(old_start=h["old_start"], old_len=h["old_len"],
+                            sha256=patch_hunks.digest(lines[h["old_start"] - 1:h["old_start"] - 1 + h["old_len"]])) for h in hunks]
+        for h, rec in zip(hunks, files[path]):
+            assert patch_hunks.digest(patch_hunks.pre_image(h)) == rec["sha256"], (path, h["old_start"])
+    out = dict(patch_sha256=patch_hunks.digest(text.splitlines()), files=files, patched_binding=patched[0],
+               stock_binding=stock[0], patched_sums=patched[1], stock_sums=stock[1])
+    with open(os.path.join(GOLD, "integration_patch_ref.json"), "w") as f:
+        json.dump(out, f, indent=1)
+        f.write("\n")
+    print("integration patch ok:", patched[1])
+
+
 if __name__ == "__main__":
-    assert os.path.isdir("/root/reference/ttt"), "the reference is only present in the build container"
+    assert REF and os.path.isdir(os.path.join(REF, "ttt")), "set TTT_VIDEO_DIT_ROOT to a checkout of the original project"
+    if len(sys.argv) > 1 and sys.argv[1] == "integration_patch":
+        gen_integration_patch()
+        sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == "sampling":
+        gen_sampling()
+        sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "transformer_layer":
         gen_transformer_layer()
         sys.exit(0)
@@ -353,5 +464,7 @@ if __name__ == "__main__":
     gen_process_input()
     gen_layer()
     gen_transformer_layer()
+    gen_sampling()
+    gen_integration_patch()
     for f in sorted(os.listdir(GOLD)):
         print(f, os.path.getsize(os.path.join(GOLD, f)))

@@ -44,9 +44,6 @@ class HostPipeline:
         self.d2h_bytes = 0
 
     def _stage(self, slot: int, host: Sequence[Optional[torch.Tensor]], first_use: bool):
-        if self.staged[slot] is None:
-            self.staged[slot] = tuple(None if t is None else torch.empty(t.shape, dtype=t.dtype, device=self.device)
-                                      for t in host)
         with torch.cuda.stream(self.s_in):
             if not first_use:
                 self.s_in.wait_event(self.ev_free[slot])
@@ -62,11 +59,16 @@ class HostPipeline:
     def run(self, batches: Iterable[Sequence[Optional[torch.Tensor]]], fn: Callable[..., torch.Tensor], host_out) -> int:
         outs = list(host_out) if isinstance(host_out, (list, tuple)) else [host_out]
         main = torch.cuda.current_stream(self.device)
-        self.s_in.wait_stream(main)  # staging buffers / earlier users of the slots are ordered before the first copy
         it = iter(batches)
         nxt = next(it, None)
         if nxt is None:
             return 0
+        if self.staged[0] is None:
+            # every slot up front: a staging block comes from the compute stream's pool and may have been freed by work still
+            # running there (an earlier op's checkpoints), so it must exist before the copy stream's wait below
+            self.staged = [tuple(None if t is None else torch.empty(t.shape, dtype=t.dtype, device=self.device) for t in nxt)
+                           for _ in range(self.depth)]
+        self.s_in.wait_stream(main)  # staging buffers / earlier users of the slots are ordered before the first copy
         self._stage(0, nxt, True)
         i = 0
         while nxt is not None:
