@@ -7,8 +7,11 @@ correctness, not only timed:
   (iii) whole scan == two half scans joined through the exported final state (forward, bit-exact) and through the
         upstream state gradient (backward, ttt_b200_mlp_backward_seeded), at NC = 804 (9 s) and 5 487 (63 s): a
         size-independent property that needs no oracle;
-  (iv)  the reference's 43-argument ttt_backward mirror == ttt_backward_simple.
+  (iv)  the reference's 43-argument ttt_backward mirror == ttt_backward_simple;
+  (v)   the per-group K-side mode == the persistent mode, batch element by batch element.
 """
+import os
+
 import pytest
 import torch
 
@@ -108,6 +111,34 @@ def test_whole_scan_equals_two_joined_halves(NC, cut):
         assert torch.equal(torch.cat([g1[i], g2[i]], dim=2), gw[i]), n
     for i, n in ((0, "dln_w"), (1, "dln_b")):
         assert O.rel_err((g1[i] + g2[i]).cpu(), gw[i].cpu()) < 1e-5, n
+
+
+def test_per_group_backward_equals_persistent_per_batch_element():
+    """The per-group K-side mode (one K-side launch per checkpoint group, ordered by host events; taken when 2*B*H + 16
+    exceeds the SM count) against the persistent mode.  H is chosen from the SM count so that B = 2 runs per group and
+    B = 1 runs persistent; NC = 37, G = 4 reuses the recompute ring and ends in a partial group.  Every sequence is
+    independent, so the B = 2 backward equals the two B = 1 backwards bit for bit, except d ln_w / d ln_b, whose sums
+    over B and over the launches run in a different order."""
+    if os.environ.get("TTT_B200_PERSISTENT", "1") == "0":
+        pytest.skip("TTT_B200_PERSISTENT=0 forces the per-group mode for every batch size")
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    H, NC, G = (sms - 16) // 2, 37, 4
+    assert tt.backward_is_persistent(H, sms) and not tt.backward_is_persistent(2 * H, sms)
+    d = _bench_like_inputs(2, H, NC, seed=7)
+    state = [d[n] for n in ("W1", "b1", "W2", "b2")]
+    fw = _forward(d, slice(0, NC), state, G)
+    both = _backward(fw, d, slice(0, NC), G)
+    out, ck, last, inputs = fw
+    one = []
+    for b in range(2):
+        pick = lambda t: t[b:b + 1].contiguous()
+        fw_b = (pick(out), [pick(c) for c in ck], [pick(w) for w in last], [pick(t) for t in inputs[:4]] + list(inputs[4:]))
+        one.append(_backward(fw_b, {"dOut": pick(d["dOut"])}, slice(0, NC), G))
+    torch.cuda.synchronize()
+    for i, n in enumerate(("dW1", "db1", "dW2", "db2", "dXQ", "dXV", "dXK", "dlast_eta"), start=2):
+        assert torch.equal(torch.cat([one[0][i], one[1][i]]), both[i]), n
+    for i, n in ((0, "dln_w"), (1, "dln_b")):
+        assert O.rel_err((one[0][i] + one[1][i]).cpu(), both[i].cpu()) < 1e-5, n
 
 
 def test_reference_43_argument_backward_matches_simple():

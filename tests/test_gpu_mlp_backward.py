@@ -52,7 +52,7 @@ def test_backward_matches_autograd_of_eager(B, H, NC, G):
 
 
 def test_backward_many_launch_units():
-    # 10 checkpoint groups of 4 -> launch units {9}, {6-8}, {3-5}, {0-2}: multi-group trajectory launches, ring-buffer reuse
+    # 10 checkpoint groups of 4 -> 10 recompute units (one group each) through the 3-slot ring: every slot is reused
     d = O.make_inputs(1, 2, 40, seed=45)
     errs = errors(d, 4)
     bad = {k: v for k, v in errs.items() if not (v < 1e-2)}

@@ -51,12 +51,12 @@ cudaError_t launch_umma_selftest(int mode, const void* A, const void* Bm, float*
 }  // namespace tb
 
 namespace tb {
+struct MlpSlot;  // recompute_ring.cuh
 bool mlp_operands_bf16();  // TTT_B200_OPERANDS=bf16: bf16 instead of fp16 operand tiles in the forward-type kernels (A/B)
 cudaError_t launch_mlp_trajectory_compact(const void* XK, const void* XV, const void* last_eta, const float* ln_w,
                                           const float* ln_b, const float* W1c, const float* b1c, const float* W2c,
                                           const float* b2c, int B, int H, int NC, int K, int G, int t0, int t_end,
-                                          uint8_t* img, float* b1img, float* b2img, int img_slots, cudaStream_t stream,
-                                          const unsigned* wait_done = nullptr);
+                                          const MlpSlot& slot, cudaStream_t stream, const unsigned* wait_done = nullptr);
 size_t mlp_backward_workspace_bytes(int B, int H, int G);
 cudaError_t launch_mlp_backward(const void* XQ, const void* XK, const void* XV, const void* last_eta, const float* ln_w,
                                 const float* ln_b, const float* W1c, const float* b1c, const float* W2c,
@@ -81,9 +81,10 @@ cudaError_t launch_linear_forward(const void* XQ, const void* XK, const void* XV
                                   const float* ln_b, const float* W1, const float* b1, float* W1c, float* b1c,
                                   float* W1o, float* b1o, void* Out, int B, int H, int NC, int ckpt_group,
                                   cudaStream_t stream);
+struct LinearImages;  // recompute_ring.cuh
 cudaError_t launch_linear_trajectory(const void* XK, const void* XV, const void* last_eta, const float* ln_w,
                                      const float* ln_b, const float* W1s, const float* b1s, long long w_stride,
-                                     long long b_stride, uint8_t* img, float* b1img, int img_slots, int B, int H, int NC,
+                                     long long b_stride, const LinearImages& out, int img_slots, int B, int H, int NC,
                                      int t0, int nsteps, cudaStream_t stream);
 size_t linear_backward_workspace_bytes(int B, int H, int NC, int G);
 cudaError_t launch_linear_backward(const void* XQ, const void* XK, const void* XV, const void* last_eta, const float* ln_w,
@@ -103,9 +104,8 @@ cudaError_t launch_attention_backward(const void* Q, const void* K, const void* 
 
 namespace tb {
 cudaError_t launch_mlp_backward_q(const CUtensorMap& tq, const CUtensorMap& tdo, const float* ln_w, const float* ln_b,
-                                  const uint8_t* img, const float* b1img, const float* b2img, uint8_t* qt, float* qb1,
-                                  float* qb2, void* dXQ, int BH, int H, int NC, int img_slots,
-                                  int G, int t0, int nsteps, cudaStream_t stream, unsigned* ready = nullptr);
+                                  const MlpSlot& slot, void* dXQ, int BH, int H, int NC, int G, int t0, int nsteps,
+                                  cudaStream_t stream, unsigned* ready = nullptr);
 }  // namespace tb
 
 namespace tb {

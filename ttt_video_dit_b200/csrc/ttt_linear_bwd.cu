@@ -25,6 +25,7 @@
 
 #include "bwd_common.cuh"
 #include "ptx.cuh"
+#include "recompute_ring.cuh"
 #include "ttt_internal.h"
 
 namespace tb {
@@ -55,14 +56,13 @@ constexpr uint32_t TM_DW = 0, TM_DZ = 64, TM_DG = 128, TM_DK0 = 192, TM_DK1 = 25
 struct LinBwdParams {
   const __nv_bfloat16* last_eta;  // [BH][NC][16]
   const float *ln_w, *ln_b;       // [H][64]
-  const uint8_t* img;             // [pairs][img_slots] x 16 KB (two stacked sequences per image, ttt_linear_fwd.cu)
-  const float* b1img;             // [pairs][img_slots][128]
+  LinearImages in;                // state images of the window, two stacked sequences per record (recompute_ring.cuh)
   float *dW1, *db1;               // carried state gradient == final output: [BH][64 f_in][64 f_out], [BH][64]
   __nv_bfloat16 *dXQ, *dXK, *dXV; // [BH][NC][16][64]
   float* dEta;                    // [BH][NC][16]
   float *dlnw, *dlnb;             // [BH][64], accumulated with atomics (pre-zeroed by the host wrapper)
   int H, NC, img_slots;
-  int t_hi, t_lo, t0;             // steps t_hi .. t_lo (descending); image of the state before step u = slot u - t0
+  int t_hi, t_lo, t0;             // steps t_hi .. t_lo (descending); image of the state before step u = record u - t0
   int first;                      // 1: start from a zero state gradient, 0: load it from dW1 / db1
   unsigned* dbg;                  // phase-timing buffer (debug builds)
 };
@@ -190,13 +190,13 @@ ttt_linear_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
   tc_fence_after();
   const uint32_t tmem = *tmem_ptr;
 
-  const uint8_t* img_g = p.img + ((size_t)(bh >> 1) * p.img_slots) * 16384 + (size_t)(bh & 1) * 8192;
-  const float* b1_g = p.b1img + ((size_t)(bh >> 1) * p.img_slots) * 128 + (bh & 1) * 64;
+  const uint8_t* img_g = p.in.image(bh >> 1, p.img_slots, 0) + (size_t)(bh & 1) * kLinSeqImageBytes;
+  const float* b1_g = p.in.image_b1(bh >> 1, p.img_slots, 0) + (bh & 1) * kLinSeqB1Floats;
   auto load_image = [&](int u) {  // state before step u -> ring slot u & 3
     const int s = u & 3;
     mbar_expect_tx(&bar_img[s], 8192 + 256);
-    bulk_load_1d(smem + SM_IMG + s * 8192, img_g + (size_t)(u - p.t0) * 16384, 8192, &bar_img[s]);
-    bulk_load_1d(b1s + s * 64, b1_g + (size_t)(u - p.t0) * 128, 256, &bar_img[s]);
+    bulk_load_1d(smem + SM_IMG + s * 8192, img_g + (size_t)(u - p.t0) * kLinImageBytes, 8192, &bar_img[s]);
+    bulk_load_1d(b1s + s * 64, b1_g + (size_t)(u - p.t0) * kLinImageB1Floats, 256, &bar_img[s]);
   };
   auto load_k = [&](int i) {  // K, V of step index i (t = t_hi - i) -> slot i % 3
     const int s = i % 3, row = (bh * NC + (p.t_hi - i)) * CS;
@@ -634,11 +634,12 @@ size_t linear_backward_window(int NC, int G) {  // steps per recompute window: a
   return (size_t)(G >= target ? G : G * (target / G));
 }
 
+// window buffers: two (recompute of window w - 1 overlaps the reverse pass over window w) unless one window covers NC
+static int linear_backward_buffers(int NC, int G) { return (size_t)NC > linear_backward_window(NC, G) ? kLinMaxBuffers : 1; }
+
 size_t linear_backward_workspace_bytes(int B, int H, int NC, int G) {
-  const size_t pairs = ((size_t)B * H + 1) / 2, slots = linear_backward_window(NC, G) + 1;
-  const size_t one = pairs * slots * (16384 + 512);
-  const size_t nwin = ((size_t)NC + linear_backward_window(NC, G) - 1) / linear_backward_window(NC, G);
-  return (nwin > 1 ? 2 : 1) * one + 1024;
+  return carve_linear_workspace(nullptr, ((size_t)B * H + 1) / 2, linear_backward_window(NC, G) + 1,
+                                linear_backward_buffers(NC, G), nullptr);
 }
 
 cudaError_t launch_linear_backward(const void* XQ, const void* XK, const void* XV, const void* last_eta, const float* ln_w,
@@ -660,14 +661,10 @@ cudaError_t launch_linear_backward(const void* XQ, const void* XK, const void* X
   const int S = (int)linear_backward_window(NC, G);
   const int nwin = (NC + S - 1) / S;
   const int K = (NC + G - 1) / G;  // checkpoints per sequence
-  const size_t pairs = ((size_t)BH + 1) / 2, slots = (size_t)S + 1;
-  const int nbuf = nwin > 1 ? 2 : 1;
-  uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
-  uint8_t* img[2];
-  float* b1img[2];
-  size_t off = 0;
-  for (int b = 0; b < nbuf; ++b) { img[b] = ws + off; off += pairs * slots * 16384; }
-  for (int b = 0; b < nbuf; ++b) { b1img[b] = reinterpret_cast<float*>(ws + off); off += pairs * slots * 512; }
+  const size_t slots = (size_t)S + 1;
+  const int nbuf = linear_backward_buffers(NC, G);
+  LinearImages img[kLinMaxBuffers];
+  carve_linear_workspace(workspace, ((size_t)BH + 1) / 2, slots, nbuf, img);
 
   std::lock_guard<std::mutex> enqueue_lock(device_enqueue_mutex());
   static bool attr_done_dev[64] = {};  // function attributes (and side streams) are per device
@@ -703,7 +700,7 @@ cudaError_t launch_linear_backward(const void* XQ, const void* XK, const void* X
     if (w + nbuf < nwin) TB_TRY(cudaStreamWaitEvent(sT, evR[b], 0), "stream wait");  // buffer still read by window w + 2
     const int ck = t0 / G;
     cudaError_t e = launch_linear_trajectory(XK, XV, last_eta, ln_w, ln_b, W1c + (size_t)ck * 64 * 64, b1c + (size_t)ck * 64,
-                                             (long long)K * 64 * 64, (long long)K * 64, img[b], b1img[b], (int)slots, B, H, NC,
+                                             (long long)K * 64 * 64, (long long)K * 64, img[b], (int)slots, B, H, NC,
                                              t0, n, sT);
     if (e != cudaSuccess) return e;
     TB_TRY(cudaEventRecord(evT[b], sT), "event record");
@@ -717,7 +714,7 @@ cudaError_t launch_linear_backward(const void* XQ, const void* XK, const void* X
     TB_TRY(cudaStreamWaitEvent(stream, evT[b], 0), "stream wait");
     linb::LinBwdParams p{};
     p.last_eta = reinterpret_cast<const __nv_bfloat16*>(last_eta);
-    p.ln_w = ln_w; p.ln_b = ln_b; p.img = img[b]; p.b1img = b1img[b];
+    p.ln_w = ln_w; p.ln_b = ln_b; p.in = img[b];
     p.dW1 = dW1; p.db1 = db1;
     p.dXQ = reinterpret_cast<__nv_bfloat16*>(dXQ); p.dXK = reinterpret_cast<__nv_bfloat16*>(dXK);
     p.dXV = reinterpret_cast<__nv_bfloat16*>(dXV); p.dEta = dEta; p.dlnw = dlnw; p.dlnb = dlnb;

@@ -16,6 +16,7 @@
 #include <stdint.h>
 
 #include "ptx.cuh"
+#include "recompute_ring.cuh"
 #include "ttt_internal.h"
 
 namespace tb {
@@ -45,12 +46,11 @@ struct LinParams {
   __nv_bfloat16* Out;             // [B,H,NC,16,64]
   int BH, H, NC, ckpt_group, K;
   // trajectory mode (backward recompute, ttt_linear_bwd.cu): run steps t0 .. t0+nsteps-1 (K side only) from the state
-  // at W1 + bh*w_stride (b1 + bh*b_stride) and save the bf16 operand image of the state BEFORE step t0+i in slot i and
-  // the state after the last step in slot nsteps: img [pairs][img_slots] x 16 KB, b1img [pairs][img_slots][128] fp32
+  // at W1 + bh*w_stride (b1 + bh*b_stride) and save the bf16 operand image of the state BEFORE step t0+i in record i and
+  // the state after the last step in record nsteps (recompute_ring.cuh)
   long long w_stride, b_stride;
   int t0, nsteps, img_slots;
-  uint8_t* img;
-  float* b1img;
+  LinearImages out;
 };
 
 template <bool kTraj>
@@ -167,10 +167,10 @@ ttt_linear_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
     float eta_i = 0.f;
     if (has_k && tok_valid && tt < 16)  // both threads of the row
       eta_i = __bfloat162float(p.last_eta[((size_t)bh_tok * p.NC + (kTraj ? p.t0 : 0) + it) * CS + tt]);
-    if (kTraj) {  // image of the state before this step (slot it; the last pass, it == nsteps, saves the final state)
-      p.b1img[((size_t)blockIdx.x * p.img_slots + it) * 128 + tid] = b1r;
+    if (kTraj) {  // image of the state before this step (record it; the last pass, it == nsteps, saves the final state)
+      p.out.image_b1(blockIdx.x, p.img_slots, it)[tid] = b1r;
       if (warp_u == 0 && elect_one()) {
-        bulk_store_1d(p.img + ((size_t)blockIdx.x * p.img_slots + it) * 16384, smem + SM_W1B, 16384);
+        bulk_store_1d(p.out.image(blockIdx.x, p.img_slots, it), smem + SM_W1B, kLinImageBytes);
         bulk_commit();
       }
       if (!has_k) break;
@@ -368,7 +368,7 @@ cudaError_t launch_linear_forward(const void* XQ, const void* XK, const void* XV
 // nsteps+1 operand images (see LinParams).  Used by launch_linear_backward (ttt_linear_bwd.cu).
 cudaError_t launch_linear_trajectory(const void* XK, const void* XV, const void* last_eta, const float* ln_w,
                                      const float* ln_b, const float* W1s, const float* b1s, long long w_stride,
-                                     long long b_stride, uint8_t* img, float* b1img, int img_slots, int B, int H, int NC,
+                                     long long b_stride, const LinearImages& out, int img_slots, int B, int H, int NC,
                                      int t0, int nsteps, cudaStream_t stream) {
   if (nsteps <= 0 || nsteps + 1 > img_slots || t0 < 0 || t0 + nsteps > NC) { g_where = "bad trajectory window"; return cudaErrorInvalidValue; }
   const uint64_t rows = (uint64_t)B * H * NC * lin::CS;
@@ -378,7 +378,7 @@ cudaError_t launch_linear_trajectory(const void* XK, const void* XV, const void*
   p.last_eta = reinterpret_cast<const __nv_bfloat16*>(last_eta);
   p.ln_w = ln_w; p.ln_b = ln_b; p.W1 = W1s; p.b1 = b1s; p.w_stride = w_stride; p.b_stride = b_stride;
   p.BH = B * H; p.H = H; p.NC = NC; p.ckpt_group = 1; p.K = 1;
-  p.t0 = t0; p.nsteps = nsteps; p.img_slots = img_slots; p.img = img; p.b1img = b1img;
+  p.t0 = t0; p.nsteps = nsteps; p.img_slots = img_slots; p.out = out;
   static bool attr_done_dev[64] = {};  // function attributes (and side streams) are per device
   bool& attr_done = *device_once(attr_done_dev);
   if (!attr_done) {

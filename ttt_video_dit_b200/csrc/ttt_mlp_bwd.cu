@@ -23,6 +23,7 @@
 
 #include "bwd_common.cuh"
 #include "ptx.cuh"
+#include "recompute_ring.cuh"
 #include "ttt_internal.h"
 
 namespace tb {
@@ -50,17 +51,10 @@ constexpr uint32_t TM_DW1 = 0;    // dW1^T accumulator, + 64*h
 constexpr uint32_t TM_DW2 = 128;  // dW2   accumulator, + 64*h
 constexpr uint32_t TM_S0 = 256, TM_S1 = 320, TM_S2 = 384, TM_S3 = 448;  // working slots of 64 columns
 
-constexpr int kRingSlots = 3;  // recompute buffers in flight (kRing of the host orchestrator)
-
 struct BwdParams {
   const __nv_bfloat16* last_eta;  // [B,H,NC,64]
   const float *ln_w, *ln_b;       // [H,64]
-  // Recompute buffers of the checkpoint groups, a ring of kRingSlots: group g (steps [g*G, (g+1)*G)) is processing unit
-  // u = K-1-g and lives in ring slot u % kRingSlots; inside a slot, step t is local index t - g*G.
-  const uint8_t* img[kRingSlots];             // [BH][img_slots] x 64 KB  {W1^T image, W2 image} of the state entering each step
-  const float *b1img[kRingSlots], *b2img[kRingSlots];  // [BH][img_slots][256], [BH][img_slots][64]
-  const uint8_t* qt[kRingSlots];              // Q-side factor tiles [BH][G] x 73728 B (ttt_mlp_bwd_q.cu)
-  const float *qb1[kRingSlots], *qb2[kRingSlots];      // Q-side contributions [BH][G][256] (d b1), [BH][G][192] = {d b2, d gamma, d beta}
+  MlpSlot ring[kRingSlots];  // recompute buffers (recompute_ring.cuh); inside a slot, step t is local index t - g*G
   float *dW1s, *dW2s, *db1s, *db2s;  // carried state gradient, fp32: [BH][256][64] x2, [BH][256], [BH][64]
   uint8_t* x2spill;                  // [BH][32 KB]
   int G, K;                          // steps per checkpoint group, number of groups
@@ -81,22 +75,8 @@ struct BwdParams {
   int dbg_group;       // group (t_lo / G) whose observer phase times are dumped
 };
 
-// Bounded spin on a device-side counter written by another kernel (acquire at gpu scope).  A protocol bug must surface as a
-// launch failure (trap), never as a hung GPU.
-static __device__ __noinline__ void wait_counter(const unsigned* ctr, unsigned want) {
-  const long long t0 = clock64();
-  for (;;) {
-    unsigned v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(ctr) : "memory");
-    if (v >= want) break;
-    __nanosleep(256);
-    if (clock64() - t0 > 20000000000LL) {
-      printf("ttt_b200: device-side flag wait timed out (block %d thread %d, have %u want %u)\n", (int)blockIdx.x, (int)threadIdx.x, v, want);
-      __trap();
-    }
-  }
-  asm volatile("fence.proxy.async;" ::: "memory");  // the data behind the flag is read by bulk / TMA loads (async proxy) too
-}
+// out of line: the wait sits in the step loop, whose code size the instruction cache decides (DESIGN.md section 4)
+static __device__ __noinline__ void wait_ready(const unsigned* flag, unsigned want) { wait_flag<256>(flag, want); }
 
 __global__ void __launch_bounds__(NT, 1)
 ttt_mlp_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
@@ -175,27 +155,27 @@ ttt_mlp_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
   // (t - 1, whose loads are issued during step t) are kept in registers and advanced once per iteration: no divisions in
   // the step loop.
   struct StepIdx { int r, l; };  // ring slot and local index inside it
-  auto step_idx = [&](int t) { const int g = t / p.G; return StepIdx{(p.K - 1 - g) % kRingSlots, t - g * p.G}; };
+  auto step_idx = [&](int t) { const int g = t / p.G; return StepIdx{ring_slot(unit_of_group(g, p.K)), t - group_begin(g, p.G)}; };
   auto step_back = [&](StepIdx& si) {  // index of the step before the one si points at
     // crossing into the previous checkpoint group = the next unit: next ring slot, last local index (every group below the
     // last one is full)
     if (si.l == 0) { si.r = (si.r + 1) % kRingSlots; si.l = p.G - 1; }
     else --si.l;
   };
-  auto img_at = [&](StepIdx si) { return p.img[si.r] + ((size_t)bh * p.img_slots + si.l) * 65536; };
-  auto qt_at = [&](StepIdx si) { return p.qt[si.r] + ((size_t)bh * p.G + si.l) * 73728; };
-  auto b1_at = [&](StepIdx si) { return p.b1img[si.r] + ((size_t)bh * p.img_slots + si.l) * HID; };
-  auto b2_at = [&](StepIdx si) { return p.b2img[si.r] + ((size_t)bh * p.img_slots + si.l) * F; };
-  auto q1_at = [&](StepIdx si) { return p.qb1[si.r] + ((size_t)bh * p.G + si.l) * HID; };
-  auto q2_at = [&](StepIdx si) { return p.qb2[si.r] + ((size_t)bh * p.G + si.l) * 192; };
+  auto img_at = [&](StepIdx si) { return p.ring[si.r].image(bh, p.img_slots, si.l); };
+  auto qt_at = [&](StepIdx si) { return p.ring[si.r].factors(bh, p.G, si.l); };
+  auto b1_at = [&](StepIdx si) { return p.ring[si.r].image_b1(bh, p.img_slots, si.l); };
+  auto b2_at = [&](StepIdx si) { return p.ring[si.r].image_b2(bh, p.img_slots, si.l); };
+  auto q1_at = [&](StepIdx si) { return p.ring[si.r].factor_b1(bh, p.G, si.l); };
+  auto q2_at = [&](StepIdx si) { return p.ring[si.r].factor_vec(bh, p.G, si.l); };
   StepIdx cur = step_idx(p.t_hi), nxt = cur;  // nxt: step t - 1 (valid while t > t_lo)
   if (p.t_hi > p.t_lo) step_back(nxt);
   // persistent mode: before the first access to the buffers of the unit that holds step t
   auto wait_unit_of = [&](int t) {
     if (p.ready == nullptr) return;
-    const int g = t / p.G, u = p.K - 1 - g;
-    const int steps = min(p.NC, (g + 1) * p.G) - g * p.G;
-    wait_counter(p.ready + (size_t)u * gridDim.x + bh, (unsigned)steps);
+    const int g = t / p.G, u = unit_of_group(g, p.K);
+    const int steps = min(p.NC, group_begin(g + 1, p.G)) - group_begin(g, p.G);
+    wait_ready(p.ready + (size_t)u * gridDim.x + bh, (unsigned)steps);
   };
   // slot roles (byte offsets of the four 32 KB hidden-lane slots); they rotate every iteration
   uint32_t sW1 = SM_HS, sA = SM_HS + 32768, sB = SM_HS + 65536, sC = SM_HS + 98304;
@@ -211,8 +191,8 @@ ttt_mlp_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
     const uint8_t* src = qt_at(t == tcur ? cur : nxt);
     mbar_expect_tx(bar_qd, 8192 + 32768 + 8192);
     tma_load_2d(smem + SM_TQ, &tmQ, 0, (int)(row_bh + (size_t)t * CS), bar_qd);
-    bulk_load_1d(smem + zs, src + 32768, 32768, bar_qd);
-    bulk_load_1d(smem + SM_TT0, src + 65536, 8192, bar_qd);
+    bulk_load_1d(smem + zs, src + kFactorDZbar1T, 32768, bar_qd);
+    bulk_load_1d(smem + SM_TT0, src + kFactorDZbar2, 8192, bar_qd);
   };
   // first iteration's loads, issued before the carried gradient is read so that both latencies overlap
   wait_unit_of(p.t_hi);
@@ -222,7 +202,7 @@ ttt_mlp_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
     mbar_expect_tx(bar_w1, 32768);
     bulk_load_1d(smem + sW1, im, 32768, bar_w1);
     mbar_expect_tx(bar_w2, 32768);
-    bulk_load_1d(smem + SM_W2I, im + 32768, 32768, bar_w2);
+    bulk_load_1d(smem + SM_W2I, im + kImageW2, 32768, bar_w2);
     mbar_expect_tx(bar_kv, 16384);
     tma_load_2d(smem + SM_TK, &tmK, 0, (int)(row_bh + (size_t)t * CS), bar_kv);
     tma_load_2d(smem + SM_TV, &tmV, 0, (int)(row_bh + (size_t)t * CS), bar_kv);
@@ -265,7 +245,7 @@ ttt_mlp_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
   if (tid < 64) {
     nb2 = b2_at(cur)[tid];
     const float* q2 = q2_at(cur);
-    nq2 = q2[tid]; nqg = q2[64 + tid]; nqb = q2[128 + tid];
+    nq2 = q2[kFactorDb2 + tid]; nqg = q2[kFactorDgamma + tid]; nqb = q2[kFactorDbeta + tid];
     if (p.t_hi < p.NC) neta = reinterpret_cast<const unsigned short*>(p.last_eta)[row_bh + (size_t)p.t_hi * CS + tid];
   }
   TICK(14);  // prologue
@@ -291,7 +271,7 @@ ttt_mlp_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
       if (tid < 64) {
         nb2 = b2_at(nxt)[tid];
         const float* q2 = q2_at(nxt);
-        nq2 = q2[tid]; nqg = q2[64 + tid]; nqb = q2[128 + tid];
+        nq2 = q2[kFactorDb2 + tid]; nqg = q2[kFactorDgamma + tid]; nqb = q2[kFactorDbeta + tid];
         neta = reinterpret_cast<const unsigned short*>(p.last_eta)[row_bh + (size_t)(t - 1) * CS + tid];
       }
     }
@@ -377,7 +357,7 @@ ttt_mlp_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
       TICK(4);
       // spill the X2 tile to L2 (needed again by the dW2 += X2^T dZ2 GEMM at the end of the K side)
       if (warp_u == 0 && elect_one()) {
-        bulk_store_1d(p.x2spill + (size_t)bh * 32768, smem + sC, 32768);
+        bulk_store_1d(p.x2spill + (size_t)bh * kX2SpillBytes, smem + sC, 32768);
         bulk_commit();
       }
       // ===== A4 [T] (all warps; thread = (row, 16 columns)): LN stats of Z2, gradZ2 -> TT1, -eta*gradZ2 -> TT2,
@@ -496,7 +476,7 @@ ttt_mlp_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         mbar_expect_tx(bar_w1r, 32768);
         bulk_load_1d(smem + sA, img_at(cur), 32768, bar_w1r);
         mbar_expect_tx(bar_x2, 32768);
-        bulk_load_1d(smem + sC, p.x2spill + (size_t)bh * 32768, 32768, bar_x2);
+        bulk_load_1d(smem + sC, p.x2spill + (size_t)bh * kX2SpillBytes, 32768, bar_x2);
       }
       // ===== A8 [T] (all warps): stage 2 = backward through the fused LN + L2 gradient (appendix B), dZ2 -> TT0, dV,
       //       d eta, +dy (= -dtarget) folded into the dK accumulator S0, column sums for d b2 / d gamma / d beta
@@ -601,7 +581,7 @@ ttt_mlp_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
       TICK(10);
       if (warp_u == 0 && (t > p.t_lo) && elect_one()) {  // the W2 image buffer is free now: fetch the next one
         mbar_expect_tx(bar_w2, 32768);
-        bulk_load_1d(smem + SM_W2I, img_at(nxt) + 32768, 32768, bar_w2);
+        bulk_load_1d(smem + SM_W2I, img_at(nxt) + kImageW2, 32768, bar_w2);
       }
       // ===== A10 [H]: dZ1 = dX2 * gelu'(Z1) + term2 -> sB ; d b1 += sum dZ1
       {
@@ -655,11 +635,7 @@ ttt_mlp_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
 
     // persistent mode: step t was the last access to its unit's recompute buffers -> the trajectory kernel that refills this
     // ring slot (unit u + kRingSlots) may start (every bulk load of the unit has completed and was consumed above)
-    if (p.done != nullptr && t % p.G == 0 && tid == 0) {
-      const int u = p.K - 1 - t / p.G;
-      __threadfence();
-      asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p.done + (size_t)u * gridDim.x + bh), "r"(1u) : "memory");
-    }
+    if (p.done != nullptr && t % p.G == 0 && tid == 0) release_flag<kSet>(p.done + (size_t)unit_of_group(t / p.G, p.K) * gridDim.x + bh);
     // next iteration's remaining loads (buffers last used by the A11 batch): K/V tiles, Q tile, dZbar1^T -> sA, dZbar2 -> TT0
     const bool more = t > p.t_lo;
     if (warp_u == 0 && (more) && elect_one()) {
@@ -754,7 +730,7 @@ __global__ void seed_state_grad_kernel(const float* __restrict__ dW1u, const flo
 }  // namespace bwd
 
 // ------------------------------------------------------------------------------------------------ host
-// Recompute state is kept in a ring of kRing buffers so that the trajectory / Q-side kernels of later units run ahead of the
+// Recompute state is kept in a ring of kRingSlots buffers (recompute_ring.cuh) so that the trajectory / Q-side kernels of later units run ahead of the
 // sequential K-side kernel (three streams).  A unit = one checkpoint group, processed last group first.
 //
 // Persistent mode (default when 2 * B*H + 16 <= SM count): ONE K-side launch walks all units; the recompute kernels run
@@ -765,14 +741,7 @@ __global__ void seed_state_grad_kernel(const float* __restrict__ dW1u, const flo
 // until the K-side CTA of its sequence releases the slot.  The SM-count condition keeps SMs free for the Q-side kernel
 // while B*H K-side CTAs and up to B*H waiting trajectory CTAs are resident (one CTA of any of the three kernels fills an
 // SM); above it the launches are ordered per unit with events as in round 1 (TTT_B200_PERSISTENT=0 forces that mode).
-constexpr int kRing = bwd::kRingSlots;
-constexpr int kMaxUnits = 4096;
-
-size_t mlp_backward_workspace_bytes(int B, int H, int G) {
-  const size_t bh = (size_t)B * H, g = (size_t)G, slots = g + 1;
-  return bh * (kRing * (slots * 65536 + slots * 256 * 4 + slots * 64 * 4) + kRing * (g * 73728 + g * 1024 + g * 768) +
-               2 * 65536 + 1024 + 256 + 32768 + 2 * (size_t)(kMaxUnits + 1) * sizeof(unsigned)) + 1024;
-}
+size_t mlp_backward_workspace_bytes(int B, int H, int G) { return carve_mlp_workspace(nullptr, (size_t)B * H, G, nullptr); }
 
 cudaError_t launch_mlp_backward(const void* XQ, const void* XK, const void* XV, const void* last_eta, const float* ln_w,
                                 const float* ln_b, const float* W1c, const float* b1c, const float* W2c,
@@ -783,26 +752,11 @@ cudaError_t launch_mlp_backward(const void* XQ, const void* XK, const void* XV, 
                                 const float* db2_last) {
   if (B <= 0 || H <= 0 || NC <= 0 || G <= 0) { g_where = "bad sizes"; return cudaErrorInvalidValue; }
   if (workspace_bytes < mlp_backward_workspace_bytes(B, H, G)) { g_where = "workspace"; return cudaErrorInvalidValue; }
-  const size_t bh = (size_t)B * H, slots = (size_t)G + 1;
+  const size_t bh = (size_t)B * H;
   const int K = (NC + G - 1) / G;  // units = checkpoint groups
   if (K > kMaxUnits) { g_where = "too many checkpoint groups"; return cudaErrorInvalidValue; }
-  uint8_t* w = reinterpret_cast<uint8_t*>(workspace);
-  w = reinterpret_cast<uint8_t*>(((uintptr_t)w + 1023) & ~(uintptr_t)1023);
-  uint8_t* img[kRing]; float *b1img[kRing], *b2img[kRing];
-  for (int i = 0; i < kRing; ++i) { img[i] = w; w += bh * slots * 65536; }
-  uint8_t* x2s = w;                      w += bh * 32768;
-  float* dW1s = reinterpret_cast<float*>(w); w += bh * 65536;
-  float* dW2s = reinterpret_cast<float*>(w); w += bh * 65536;
-  for (int i = 0; i < kRing; ++i) { b1img[i] = reinterpret_cast<float*>(w); w += bh * slots * 1024; }
-  for (int i = 0; i < kRing; ++i) { b2img[i] = reinterpret_cast<float*>(w); w += bh * slots * 256; }
-  float* db1s = reinterpret_cast<float*>(w); w += bh * 1024;
-  float* db2s = reinterpret_cast<float*>(w); w += bh * 256;
-  uint8_t* qt[kRing]; float *qb1[kRing], *qb2[kRing];   // Q-side factor tiles / vectors of a group
-  for (int i = 0; i < kRing; ++i) { qt[i] = w; w += bh * (size_t)G * 73728; }
-  for (int i = 0; i < kRing; ++i) { qb1[i] = reinterpret_cast<float*>(w); w += bh * (size_t)G * 1024; }
-  for (int i = 0; i < kRing; ++i) { qb2[i] = reinterpret_cast<float*>(w); w += bh * (size_t)G * 768; }
-  unsigned* ready = reinterpret_cast<unsigned*>(w); w += bh * (size_t)(kMaxUnits + 1) * sizeof(unsigned);  // [unit][bh]
-  unsigned* done = reinterpret_cast<unsigned*>(w);  w += bh * (size_t)(kMaxUnits + 1) * sizeof(unsigned);
+  MlpWorkspace ws;
+  carve_mlp_workspace(workspace, bh, G, &ws);
 
   CUtensorMap tq, tk, tv, tdo;
   const uint64_t rows = (uint64_t)bh * NC * 64;
@@ -826,7 +780,7 @@ cudaError_t launch_mlp_backward(const void* XQ, const void* XK, const void* XV, 
   // three streams per device (created once): T = trajectory, Q = Q-side kernel, main = sequential K-side kernel
   struct Side {
     cudaStream_t sT = nullptr, sQ = nullptr;
-    cudaEvent_t fork = nullptr, joinT = nullptr, joinQ = nullptr, evT[kRing] = {}, evQ[kRing] = {}, evR[kRing] = {};
+    cudaEvent_t fork = nullptr, joinT = nullptr, joinQ = nullptr, evT[kRingSlots] = {}, evQ[kRingSlots] = {}, evR[kRingSlots] = {};
   };
   static Side sides[64];
   Side& sd = sides[dev & 63];
@@ -838,7 +792,7 @@ cudaError_t launch_mlp_backward(const void* XQ, const void* XK, const void* XV, 
     TB_TRY(cudaEventCreateWithFlags(&sd.fork, cudaEventDisableTiming), "event");
     TB_TRY(cudaEventCreateWithFlags(&sd.joinT, cudaEventDisableTiming), "event");
     TB_TRY(cudaEventCreateWithFlags(&sd.joinQ, cudaEventDisableTiming), "event");
-    for (int i = 0; i < kRing; ++i) {
+    for (int i = 0; i < kRingSlots; ++i) {
       TB_TRY(cudaEventCreateWithFlags(&sd.evT[i], cudaEventDisableTiming), "event");
       TB_TRY(cudaEventCreateWithFlags(&sd.evQ[i], cudaEventDisableTiming), "event");
       TB_TRY(cudaEventCreateWithFlags(&sd.evR[i], cudaEventDisableTiming), "event");
@@ -849,72 +803,69 @@ cudaError_t launch_mlp_backward(const void* XQ, const void* XK, const void* XV, 
   const bool persistent = persistent_env != 0 && 2 * (int)bh + 16 <= sm_count_dev[dev & 63];
   const bool seeded = dW1_last != nullptr;
   if (seeded) {  // carried gradient starts from the upstream d/dW_last instead of zero
-    bwd::seed_state_grad_kernel<<<(unsigned)bh, 256, 0, stream>>>(dW1_last, db1_last, dW2_last, db2_last, dW1s, dW2s, db1s, db2s);
+    bwd::seed_state_grad_kernel<<<(unsigned)bh, 256, 0, stream>>>(dW1_last, db1_last, dW2_last, db2_last, ws.dW1s, ws.dW2s, ws.db1s,
+                                                                   ws.db2s);
     TB_TRY(cudaGetLastError(), "seed launch");
   }
   if (persistent) {
-    TB_TRY(cudaMemsetAsync(ready, 0, bh * (size_t)K * sizeof(unsigned), stream), "memset ready flags");
-    TB_TRY(cudaMemsetAsync(done, 0, bh * (size_t)K * sizeof(unsigned), stream), "memset done flags");
+    TB_TRY(cudaMemsetAsync(ws.ready, 0, bh * (size_t)K * sizeof(unsigned), stream), "memset ready flags");
+    TB_TRY(cudaMemsetAsync(ws.done, 0, bh * (size_t)K * sizeof(unsigned), stream), "memset done flags");
   }
-  // unit u = group K-1-u -> ring buffer r = u % kRing: trajectory (images of W_{t0} .. W_{t1}) on stream T, then the Q-side
-  // kernel (steps t0 .. t1-1) on stream Q
+  // unit u: trajectory (images of W_{t0} .. W_{t1}) on stream T, then the Q-side kernel (steps t0 .. t1-1) on stream Q
   auto recompute = [&](int u) -> cudaError_t {
-    const int r = u % kRing, g = K - 1 - u;
-    const int t0 = g * G, t1 = ((g + 1) * G < NC) ? (g + 1) * G : NC;
-    const unsigned* wait_done = (persistent && u >= kRing) ? done + (size_t)(u - kRing) * bh : nullptr;
+    const int r = ring_slot(u), g = unit_of_group(u, K);
+    const int t0 = group_begin(g, G), t1 = group_end(g, G, NC);
+    const unsigned* wait_done = (persistent && u >= kRingSlots) ? ws.done + (size_t)(u - kRingSlots) * bh : nullptr;
     cudaError_t e = launch_mlp_trajectory_compact(XK, XV, last_eta, ln_w, ln_b, W1c, b1c, W2c, b2c, B, H, NC, K, G, t0, t1,
-                                                  img[r], b1img[r], b2img[r], (int)slots, sd.sT, wait_done);
+                                                  ws.ring[r], sd.sT, wait_done);
     if (e != cudaSuccess) return e;
     if ((e = cudaEventRecord(sd.evT[r], sd.sT)) != cudaSuccess) return e;
     if ((e = cudaStreamWaitEvent(sd.sQ, sd.evT[r], 0)) != cudaSuccess) return e;
-    e = launch_mlp_backward_q(tq, tdo, ln_w, ln_b, img[r], b1img[r], b2img[r], qt[r], qb1[r], qb2[r], dXQ,
-                              (int)bh, H, NC, (int)slots, G, t0, t1 - t0, sd.sQ, persistent ? ready + (size_t)u * bh : nullptr);
+    e = launch_mlp_backward_q(tq, tdo, ln_w, ln_b, ws.ring[r], dXQ, (int)bh, H, NC, G, t0, t1 - t0, sd.sQ,
+                              persistent ? ws.ready + (size_t)u * bh : nullptr);
     if (e != cudaSuccess) return e;
     return cudaEventRecord(sd.evQ[r], sd.sQ);
   };
   bwd::BwdParams p{};
   p.last_eta = reinterpret_cast<const __nv_bfloat16*>(last_eta);
   p.ln_w = ln_w; p.ln_b = ln_b;
-  for (int i = 0; i < kRing; ++i) {
-    p.img[i] = img[i]; p.b1img[i] = b1img[i]; p.b2img[i] = b2img[i];
-    p.qt[i] = qt[i]; p.qb1[i] = qb1[i]; p.qb2[i] = qb2[i];
-  }
-  p.dW1s = dW1s; p.dW2s = dW2s; p.db1s = db1s; p.db2s = db2s;
-  p.x2spill = x2s;
+  for (int i = 0; i < kRingSlots; ++i) p.ring[i] = ws.ring[i];
+  p.dW1s = ws.dW1s; p.dW2s = ws.dW2s; p.db1s = ws.db1s; p.db2s = ws.db2s;
+  p.x2spill = ws.x2spill;
   p.G = G; p.K = K;
   p.dXQ = reinterpret_cast<__nv_bfloat16*>(dXQ); p.dXK = reinterpret_cast<__nv_bfloat16*>(dXK);
   p.dXV = reinterpret_cast<__nv_bfloat16*>(dXV); p.dEta = reinterpret_cast<__nv_bfloat16*>(dEta);
   p.dlnw = dlnw; p.dlnb = dlnb;
   p.dW1 = dW1; p.db1 = db1; p.dW2 = dW2; p.db2 = db2;
-  p.H = H; p.NC = NC; p.img_slots = (int)slots;
+  p.H = H; p.NC = NC; p.img_slots = G + 1;
   p.dbg_group = dbg_group_env;
   p.dbg = g_timing_buf;  // observers: the launch whose t_lo / G equals TTT_DBG_GROUP; per-launch stamps are kept
 
   TB_TRY(cudaEventRecord(sd.fork, stream), "fork record");
   TB_TRY(cudaStreamWaitEvent(sd.sT, sd.fork, 0), "fork wait");
   TB_TRY(cudaStreamWaitEvent(sd.sQ, sd.fork, 0), "fork wait");
-  for (int i = 0; i < kRing && i < K; ++i) TB_TRY(recompute(i), "trajectory / Q launch");
+  for (int i = 0; i < kRingSlots && i < K; ++i) TB_TRY(recompute(i), "trajectory / Q launch");
 
   if (persistent) {
     p.t_hi = NC - 1; p.t_lo = 0;
     p.first = seeded ? 0 : 1;
-    p.ready = ready; p.done = done;
+    p.ready = ws.ready; p.done = ws.done;
     bwd::ttt_mlp_bwd_kernel<<<(unsigned)bh, bwd::NT, bwd::SM_TOTAL, stream>>>(tq, tk, tv, p);
     TB_TRY(cudaGetLastError(), "reverse launch (persistent)");
-    for (int u = kRing; u < K; ++u) TB_TRY(recompute(u), "trajectory / Q launch");  // each waits on-device for its ring slot
+    for (int u = kRingSlots; u < K; ++u) TB_TRY(recompute(u), "trajectory / Q launch");  // each waits on-device for its ring slot
   } else {
     for (int u = 0; u < K; ++u) {
-      const int r = u % kRing, g = K - 1 - u;
+      const int r = ring_slot(u), g = unit_of_group(u, K);
       TB_TRY(cudaStreamWaitEvent(stream, sd.evQ[r], 0), "wait Q-side");
-      p.t_hi = (((g + 1) * G < NC) ? (g + 1) * G : NC) - 1;
-      p.t_lo = g * G;
+      p.t_hi = group_end(g, G, NC) - 1;
+      p.t_lo = group_begin(g, G);
       p.first = (u == 0 && !seeded) ? 1 : 0;
       bwd::ttt_mlp_bwd_kernel<<<(unsigned)bh, bwd::NT, bwd::SM_TOTAL, stream>>>(tq, tk, tv, p);
       TB_TRY(cudaGetLastError(), "reverse launch");
-      if (u + kRing < K) {  // ring buffer r is free again once this launch is done: recompute unit u + kRing into it
+      if (u + kRingSlots < K) {  // ring buffer r is free again once this launch is done: recompute unit u + kRingSlots into it
         TB_TRY(cudaEventRecord(sd.evR[r], stream), "record reverse");
         TB_TRY(cudaStreamWaitEvent(sd.sT, sd.evR[r], 0), "wait reverse");
-        TB_TRY(recompute(u + kRing), "trajectory / Q launch");
+        TB_TRY(recompute(u + kRingSlots), "trajectory / Q launch");
       }
     }
   }

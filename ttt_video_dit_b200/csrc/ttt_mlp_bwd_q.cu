@@ -16,6 +16,7 @@
 
 #include "bwd_common.cuh"
 #include "ptx.cuh"
+#include "recompute_ring.cuh"
 #include "ttt_internal.h"
 
 namespace tb {
@@ -34,12 +35,9 @@ constexpr uint32_t QT_S0 = 0, QT_S1 = 64, QT_S2 = 128;  // TMEM working slots (2
 
 struct BwdQParams {
   const float *ln_w, *ln_b;      // [H,64]
-  const uint8_t* img;            // [BH][img_slots] x 64 KB
-  const float *b1img, *b2img;    // [BH][img_slots][256], [BH][img_slots][64]
-  uint8_t* qt;                   // out: [BH][G] x 73728 B  { Xbar2^T 32 KB, dZbar1^T 32 KB, dZbar2 8 KB }
-  float *qb1, *qb2;              // out: [BH][G][256] (sum_i dZbar1), [BH][G][192] = {sum_i dZbar2, d gamma, d beta of the step}
+  MlpSlot slot;                  // reads the state images, writes the factor records (recompute_ring.cuh)
   __nv_bfloat16* dXQ;            // out
-  int H, NC, img_slots, G, t0;   // step s = t0 + blockIdx.x uses image slot blockIdx.x + 1
+  int H, NC, img_slots, G, t0;   // step s = t0 + blockIdx.x reads image record blockIdx.x + 1
   unsigned* ready;               // persistent K-side mode: counter [BH] of this unit, +1 per finished CTA (may be null)
 };
 
@@ -97,24 +95,25 @@ ttt_mlp_bwd_q_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
     tma_prefetch_desc(&tmQ); tma_prefetch_desc(&tmDO);
   }
   if (warp == 0) tmem_alloc<256>(tmem_ptr);
-  const size_t slot = (size_t)bh * p.img_slots + (sl + 1);
+  const float* b2rec = p.slot.image_b2(bh, p.img_slots, sl + 1);
+  const float* b1rec = p.slot.image_b1(bh, p.img_slots, sl + 1);
   if (tid < 64) {
     lnw[tid] = p.ln_w[head * 64 + tid];
     lnb[tid] = p.ln_b[head * 64 + tid];
-    b2t[tid] = p.b2img[slot * 64 + tid];
+    b2t[tid] = b2rec[tid];
     cb2[tid] = 0.f; cgam[tid] = 0.f; cbet[tid] = 0.f;
   }
-  const float b1t = p.b1img[slot * 256 + j];
+  const float b1t = b1rec[j];
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = *tmem_ptr;
   const size_t row = ((size_t)bh * p.NC + s) * 64;
   if (warp_u == 0 && elect_one()) {
-    const uint8_t* im = p.img + slot * 65536;
-    mbar_expect_tx(bar_w, 65536);
-    bulk_load_1d(smem + QS_W1I, im, 32768, bar_w);
-    bulk_load_1d(smem + QS_W2I, im + 32768, 32768, bar_w);
+    const uint8_t* im = p.slot.image(bh, p.img_slots, sl + 1);
+    mbar_expect_tx(bar_w, kImageBytes);
+    bulk_load_1d(smem + QS_W1I, im + kImageW1T, 32768, bar_w);
+    bulk_load_1d(smem + QS_W2I, im + kImageW2, 32768, bar_w);
     mbar_expect_tx(bar_qd, 16384);
     tma_load_2d(smem + QS_TQ, &tmQ, 0, (int)row, bar_qd);
     tma_load_2d(smem + QS_TDO, &tmDO, 0, (int)row, bar_qd);
@@ -221,7 +220,7 @@ ttt_mlp_bwd_q_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
       acc += ((v[0] + v[1]) + (v[2] + v[3])) + ((v[4] + v[5]) + (v[6] + v[7]));
       st_shared_v4(sbase + QS_ZB + sw128_off(j, c), pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7]));
     }
-    p.qb1[((size_t)bh * p.G + sl) * 256 + j] = acc;
+    p.slot.factor_b1(bh, p.G, sl)[j] = acc;
   }
   PHASE_SYNC();
   // ===== Q7 MMA: dQ_u = dZbar1 . W1 -> S2 ; factor tiles -> global scratch
@@ -229,19 +228,19 @@ ttt_mlp_bwd_q_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
     tc_fence_after();
     mma_tok_rolled(tmem + QT_S2, sbase + QS_ZB, sbase + QS_W1I);
     tc_commit(mma_bar);
-    uint8_t* dst = p.qt + ((size_t)bh * p.G + sl) * 73728;
-    bulk_store_1d(dst, smem + QS_XB, 32768);
-    bulk_store_1d(dst + 32768, smem + QS_ZB, 32768);
-    bulk_store_1d(dst + 65536, smem + QS_TT0, 8192);
+    uint8_t* dst = p.slot.factors(bh, p.G, sl);
+    bulk_store_1d(dst + kFactorXbar2T, smem + QS_XB, 32768);
+    bulk_store_1d(dst + kFactorDZbar1T, smem + QS_ZB, 32768);
+    bulk_store_1d(dst + kFactorDZbar2, smem + QS_TT0, 8192);
     bulk_commit();
   }
   if (tid < 64) {
     // per-step partials, added by the sequential K-side kernel in step order (no global atomics: the LayerNorm parameter
     // gradients are bitwise reproducible); the shared-memory sums above start from zero and take exactly two addends
-    float* q2 = p.qb2 + ((size_t)bh * p.G + sl) * 192;
-    q2[tid] = cb2[tid];
-    q2[64 + tid] = cgam[tid];
-    q2[128 + tid] = cbet[tid];
+    float* q2 = p.slot.factor_vec(bh, p.G, sl);
+    q2[kFactorDb2 + tid] = cb2[tid];
+    q2[kFactorDgamma + tid] = cgam[tid];
+    q2[kFactorDbeta + tid] = cbet[tid];
   }
   MMA_WAIT();
   // ===== Q8 [T]: dQ = dO + dQ_u
@@ -258,19 +257,15 @@ ttt_mlp_bwd_q_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
   if (warp_u == 0 && elect_one()) bulk_wait<0>();
   tc_fence_before();
   __syncthreads();
-  if (p.ready != nullptr && tid == 0) {  // every thread's global stores precede the barrier above; release them at gpu scope
-    __threadfence();
-    asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p.ready + bh), "r"(1u) : "memory");
-  }
+  if (p.ready != nullptr && tid == 0) release_flag<kCount>(p.ready + bh);  // every thread's global stores precede the barrier above
   if (warp == 0) tmem_dealloc<256>(tmem);
 }
 
 }  // namespace bwd
 
 cudaError_t launch_mlp_backward_q(const CUtensorMap& tq, const CUtensorMap& tdo, const float* ln_w, const float* ln_b,
-                                  const uint8_t* img, const float* b1img, const float* b2img, uint8_t* qt, float* qb1,
-                                  float* qb2, void* dXQ, int BH, int H, int NC, int img_slots,
-                                  int G, int t0, int nsteps, cudaStream_t stream, unsigned* ready) {
+                                  const MlpSlot& slot, void* dXQ, int BH, int H, int NC, int G, int t0, int nsteps,
+                                  cudaStream_t stream, unsigned* ready) {
   static bool attr_done_dev[64] = {};  // function attributes (and side streams) are per device
   bool& attr_done = *device_once(attr_done_dev);
   if (!attr_done) {
@@ -278,9 +273,8 @@ cudaError_t launch_mlp_backward_q(const CUtensorMap& tq, const CUtensorMap& tdo,
     attr_done = true;
   }
   bwd::BwdQParams p{};
-  p.ln_w = ln_w; p.ln_b = ln_b; p.img = img; p.b1img = b1img; p.b2img = b2img;
-  p.qt = qt; p.qb1 = qb1; p.qb2 = qb2; p.dXQ = reinterpret_cast<__nv_bfloat16*>(dXQ);
-  p.H = H; p.NC = NC; p.img_slots = img_slots; p.G = G; p.t0 = t0; p.ready = ready;
+  p.ln_w = ln_w; p.ln_b = ln_b; p.slot = slot; p.dXQ = reinterpret_cast<__nv_bfloat16*>(dXQ);
+  p.H = H; p.NC = NC; p.img_slots = G + 1; p.G = G; p.t0 = t0; p.ready = ready;
   dim3 grid(nsteps, BH);
   bwd::ttt_mlp_bwd_q_kernel<<<grid, 256, bwd::QS_TOTAL, stream>>>(tq, tdo, p);
   return cudaGetLastError();

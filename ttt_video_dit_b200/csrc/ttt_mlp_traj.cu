@@ -1,7 +1,7 @@
-// TTT-MLP trajectory recompute for the backward pass (sm_100a): replays the K side of steps [t0, t0+n) of one
-// checkpoint group from the checkpointed fp32 state and saves the bf16 operand image of the state entering every step
-// (what ttt-tk/kernels/ttt_backward/ttt.cu:1-260 re-materialises per group from its W checkpoints).  Same arithmetic
-// and tile conventions as ttt_mlp_fwd.cu (K side only), but written for CODE SIZE, not speed:
+// TTT-MLP trajectory recompute for the backward pass (sm_100a): replays the K side of the steps of one checkpoint group
+// from the checkpointed fp32 state and saves the bf16 operand image of the state entering every step (what
+// ttt-tk/kernels/ttt_backward/ttt.cu:1-260 re-materialises per group from its W checkpoints).  Same arithmetic and tile
+// conventions as ttt_mlp_fwd.cu (K side only), but written for CODE SIZE, not speed:
 //
 // The backward pass runs three kernels concurrently (this one, the parallel Q-side kernel and the sequential K-side
 // kernel).  Measured on B200 (profiles/r01_icache_interference_*.log): a co-running kernel whose loop body exceeds the
@@ -22,6 +22,7 @@
 
 #include "bwd_common.cuh"
 #include "ptx.cuh"
+#include "recompute_ring.cuh"
 #include "ttt_internal.h"
 
 namespace tb {
@@ -87,11 +88,8 @@ struct TrajParams {
   const __nv_bfloat16* last_eta;        // [B,H,NC,64]
   const float *ln_w, *ln_b;             // [H,64]
   const float *W1, *b1, *W2, *b2;       // checkpoint arrays [BH][K]...
-  // one launch covers the steps [t0, t_end) of nsub = gridDim.y consecutive checkpoint groups of G steps: CTA (bh, sub)
-  // replays group sub from its own checkpoint (index t0 / G + sub) into the image slots sub * G ...
-  int NC, H, K, G, t0, t_end, img_slots;
-  uint8_t* img;                         // [BH][img_slots] x 64 KB
-  float *b1img, *b2img;                 // [BH][img_slots][256], [BH][img_slots][64]
+  int NC, H, K, G, t0, t_end, img_slots;  // one checkpoint group: steps [t0, t_end), t0 = checkpoint index * G
+  MlpSlot slot;                         // receives the images of the states entering steps t0 .. t_end (recompute_ring.cuh)
   // persistent K-side mode: [BH] flags of the unit that used this ring slot before; the CTA of sequence bh starts writing
   // only after the K-side CTA of bh has released the slot (null: the host orders the launches with events instead)
   const unsigned* wait_done;
@@ -105,28 +103,12 @@ ttt_mlp_traj_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_consta
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int warp_u = uniform_warp_id();  // == warp, provably warp-uniform: single-thread issue blocks branch on it
   const int bh = blockIdx.x, head = bh % p.H;
-  const int sub = blockIdx.y;
-  const int my_t0 = p.t0 + sub * p.G;
-  const int n = (my_t0 + p.G < p.t_end) ? p.G : p.t_end - my_t0;
-  // the state after the last step of a group is the next group's checkpoint: only the last group of the launch stores it
-  const bool store_last = (sub == (int)gridDim.y - 1);
+  const int n = p.t_end - p.t0;
   const int half = warp >> 2, j = tid;
   const uint32_t lane_addr = ((uint32_t)((warp & 3) * 32)) << 16;
 
-  if (p.wait_done != nullptr) {  // bounded spin (trap on timeout): a protocol bug must not hang the GPU
-    if (tid == 0) {
-      const long long t0c = clock64();
-      for (;;) {
-        unsigned v;
-        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p.wait_done + bh) : "memory");
-        if (v != 0) break;
-        __nanosleep(512);
-        if (clock64() - t0c > 20000000000LL) {
-          printf("ttt_b200: trajectory kernel timed out waiting for its ring slot (block %d)\n", (int)blockIdx.x);
-          __trap();
-        }
-      }
-    }
+  if (p.wait_done != nullptr) {
+    if (tid == 0) wait_flag<512>(p.wait_done + bh, 1);
     __syncthreads();
   }
   float* b2s = reinterpret_cast<float*>(smem + SM_MISC);
@@ -149,7 +131,7 @@ ttt_mlp_traj_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_consta
     tma_prefetch_desc(&tmV);
   }
   if (warp == 0) tmem_alloc<512>(tmem_ptr);
-  const size_t st = (size_t)bh * p.K + (size_t)(my_t0 / p.G);
+  const size_t st = (size_t)bh * p.K + (size_t)(p.t0 / p.G);
   if (tid < 64) {
     lnw[tid] = p.ln_w[head * 64 + tid];
     lnb[tid] = p.ln_b[head * 64 + tid];
@@ -160,11 +142,10 @@ ttt_mlp_traj_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_consta
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = *tmem_ptr;
-  const size_t row_base = ((size_t)bh * p.NC + my_t0) * CS;
-  const size_t slot0 = (size_t)bh * p.img_slots + (size_t)sub * p.G;
-  uint8_t* img = p.img + slot0 * 65536;
-  float* b1img = p.b1img + slot0 * HID;
-  float* b2img = p.b2img + slot0 * F;
+  const size_t row_base = ((size_t)bh * p.NC + p.t0) * CS;
+  uint8_t* img = p.slot.image(bh, p.img_slots, 0);
+  float* b1img = p.slot.image_b1(bh, p.img_slots, 0);
+  float* b2img = p.slot.image_b2(bh, p.img_slots, 0);
 
   if (warp_u == 0 && elect_one()) {
     mbar_expect_tx(&tma_bar[0], 16384);
@@ -172,7 +153,7 @@ ttt_mlp_traj_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_consta
     tma_load_2d(smem + SM_V, &tmV, 0, (int)row_base, &tma_bar[0]);
   }
 
-  // ---- checkpointed state -> TMEM accumulators + bf16 operand copies (= image slot 0)
+  // ---- checkpointed state -> TMEM accumulators + bf16 operand copies (= image record 0)
   float b1r = p.b1[st * HID + j];
   {
     const float* W1g = p.W1 + st * F * HID;
@@ -184,12 +165,12 @@ ttt_mlp_traj_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_consta
       for (int i = 0; i < 16; ++i) v[i] = W1g[(size_t)(16 * c + i) * HID + j];
       tmem_st16(tmem + lane_addr + TM_W1 + 64 * half + 16 * c, reinterpret_cast<uint32_t*>(v));
       st_row16_op<kF16>(sbase + SM_W1B, j, 2 * c, v);
-      st_image16(img, j, 2 * c, v);  // image of the state entering step t0 (slot 0)
+      st_image16(img + kImageW1T, j, 2 * c, v);  // image of the state entering step t0
 #pragma unroll
       for (int i = 0; i < 16; ++i) v[i] = W2g[(size_t)j * F + 16 * c + i];
       tmem_st16(tmem + lane_addr + TM_W2 + 64 * half + 16 * c, reinterpret_cast<uint32_t*>(v));
       st_row16_op<kF16>(sbase + SM_W2B, j, 2 * c, v);
-      st_image16(img + 32768, j, 2 * c, v);
+      st_image16(img + kImageW2, j, 2 * c, v);
     }
     b1img[j] = b1r;
     if (tid < 64) b2img[tid] = b2s[tid];
@@ -401,16 +382,16 @@ ttt_mlp_traj_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_consta
     mma_phase ^= 1;
     tc_fence_after();
 
-    // ---- P8: operand copies of the new state (smem) + its bf16 image (global) = image slot it + 1
-    const bool store_img = store_last || it + 1 < n;
-    uint8_t* img_n = img + (size_t)(it + 1) * 65536;
+    // ---- P8: operand copies of the new state (smem) + its bf16 image (global) = image record it + 1 (the last one is
+    //          the next group's checkpoint, read by the Q-side kernel of step t_end - 1)
+    uint8_t* img_n = img + (size_t)(it + 1) * kImageBytes;
 #pragma unroll 1
     for (int c = 0; c < 4; ++c) {
       float v[16];
       tmem_ld16(tmem + lane_addr + TM_W1 + 64 * half + 16 * c, reinterpret_cast<uint32_t*>(v));
       tc_wait_ld();
       st_row16_op<kF16>(sbase + SM_W1B, j, 2 * c, v);
-      if (store_img) st_image16(img_n, j, 2 * c, v);
+      st_image16(img_n + kImageW1T, j, 2 * c, v);
     }
     if (kF16 && it + 1 < n) {  // next step's K tile (TMA issued at the top of this step): bf16 -> f16 in place
       mbar_wait(&tma_bar[slot ^ 1], ((it + 1) >> 1) & 1);
@@ -426,12 +407,10 @@ ttt_mlp_traj_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_consta
       tmem_ld16(tmem + lane_addr + TM_W2 + 64 * half + 16 * c, reinterpret_cast<uint32_t*>(v));
       tc_wait_ld();
       st_row16_op<kF16>(sbase + SM_W2B, j, 2 * c, v);
-      if (store_img) st_image16(img_n + 32768, j, 2 * c, v);
+      st_image16(img_n + kImageW2, j, 2 * c, v);
     }
-    if (store_img) {
-      b1img[(size_t)(it + 1) * HID + j] = b1r;
-      if (tid < 64) b2img[(size_t)(it + 1) * F + tid] = b2s[tid];  // b2s was updated by the same thread in P6
-    }
+    b1img[(size_t)(it + 1) * kImageB1Floats + j] = b1r;
+    if (tid < 64) b2img[(size_t)(it + 1) * kImageB2Floats + tid] = b2s[tid];  // b2s was updated by the same thread in P6
     fence_proxy_async();
     tc_fence_before();
     __syncthreads();
@@ -447,10 +426,9 @@ ttt_mlp_traj_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_consta
 cudaError_t launch_mlp_trajectory_compact(const void* XK, const void* XV, const void* last_eta, const float* ln_w,
                                           const float* ln_b, const float* W1c, const float* b1c, const float* W2c,
                                           const float* b2c, int B, int H, int NC, int K, int G, int t0, int t_end,
-                                          uint8_t* img, float* b1img, float* b2img, int img_slots, cudaStream_t stream,
-                                          const unsigned* wait_done) {
-  if (G <= 0 || t0 % G != 0 || t_end <= t0 || t_end > NC || t_end - t0 + 1 > img_slots) {
-    g_where = "bad trajectory window";
+                                          const MlpSlot& slot, cudaStream_t stream, const unsigned* wait_done) {
+  if (G <= 0 || t0 < 0 || t0 >= NC || t0 % G != 0 || t_end != group_end(t0 / G, G, NC)) {
+    g_where = "trajectory window is not one checkpoint group";
     return cudaErrorInvalidValue;
   }
   const uint64_t rows = (uint64_t)B * H * NC * traj::CS;
@@ -459,8 +437,8 @@ cudaError_t launch_mlp_trajectory_compact(const void* XK, const void* XV, const 
   traj::TrajParams p{};
   p.last_eta = reinterpret_cast<const __nv_bfloat16*>(last_eta);
   p.ln_w = ln_w; p.ln_b = ln_b; p.W1 = W1c; p.b1 = b1c; p.W2 = W2c; p.b2 = b2c;
-  p.NC = NC; p.H = H; p.K = K; p.G = G; p.t0 = t0; p.t_end = t_end; p.img_slots = img_slots;
-  p.img = img; p.b1img = b1img; p.b2img = b2img; p.wait_done = wait_done;
+  p.NC = NC; p.H = H; p.K = K; p.G = G; p.t0 = t0; p.t_end = t_end; p.img_slots = G + 1;
+  p.slot = slot; p.wait_done = wait_done;
   static bool attr_done_dev[64] = {};  // function attributes (and side streams) are per device
   bool& attr_done = *device_once(attr_done_dev);
   if (!attr_done) {
@@ -469,9 +447,8 @@ cudaError_t launch_mlp_trajectory_compact(const void* XK, const void* XV, const 
     attr_done = true;
   }
   g_where = "trajectory launch";
-  const dim3 grid(B * H, (t_end - t0 + G - 1) / G);
-  if (mlp_operands_bf16()) traj::ttt_mlp_traj_kernel<false><<<grid, traj::NT, traj::SM_TOTAL, stream>>>(tk, tv, p);
-  else                     traj::ttt_mlp_traj_kernel<true><<<grid, traj::NT, traj::SM_TOTAL, stream>>>(tk, tv, p);
+  if (mlp_operands_bf16()) traj::ttt_mlp_traj_kernel<false><<<B * H, traj::NT, traj::SM_TOTAL, stream>>>(tk, tv, p);
+  else                     traj::ttt_mlp_traj_kernel<true><<<B * H, traj::NT, traj::SM_TOTAL, stream>>>(tk, tv, p);
   return cudaGetLastError();
 }
 
